@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the v2e hot path on B200 (see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference_cuda]
-                    [--workload headline|s|c3|c5]
+                    [--workload headline|s|c3|c5] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json: "Mevents/s + interpolated-frames/s ... 1280x720 at 10x slowdown"):
 one clip of 9 source frames (1280x720 uint8, smooth random texture translating 10 px per source
@@ -23,6 +23,9 @@ Secondary lines in the same JSON object (BASELINE.json configs, SURVEY.md 8d):
                           bands, centre-surround pixel model sharded over pixel rows (halo exchange per Euler chunk)
 `--impl reference` times the UNMODIFIED reference (oracle/_ref: the vendored v2ecore package) on the host cores.
 One JSON line on stdout (rank 0).
+`--dump-outputs DIR` (headline, rank 0) writes the events, frame offsets and frame times of the last timed step as
+DIR/<name>.npy (bench.dump_outputs). Every input is seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import ctypes
@@ -135,6 +138,30 @@ def unet_activation_bytes(in_ch, out_ch, H, W, B):
         outb = 32 if i == len(layers) - 1 else pad16(co) * 2
         tot += B * (H >> lvl) * (W >> lvl) * (inb + outb)
     return tot
+
+
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, events, offsets, times, budget=DUMP_BYTES, seed=0):
+    """--dump-outputs: what V2EPipeline.run returned for one clip, as <out_dir>/<name>.npy: events [M, 4] float32
+    (t, x, y, p), offsets [T+1] and times [T] (float64). The order in which the pixel model emits the rows of one
+    frame varies from run to run, so each frame's rows are written sorted by (t, y, x, p). When the files would
+    exceed `budget` bytes, events is a seeded sample of those rows, kept in order, and events_rows [k] (float64)
+    holds their row numbers."""
+    os.makedirs(out_dir, exist_ok=True)
+    ev = np.asarray(events, np.float32)
+    frame = np.repeat(np.arange(len(offsets) - 1), np.diff(offsets))
+    ev = ev[np.lexsort((ev[:, 3], ev[:, 1], ev[:, 2], ev[:, 0], frame))]
+    out = {"offsets": np.asarray(offsets, np.float64), "times": np.asarray(times, np.float64)}
+    room = budget - sum(a.nbytes for a in out.values()) - 4 * 4096        # .npy headers
+    if ev.nbytes > room:
+        rows = np.sort(np.random.default_rng(seed).choice(len(ev), room // (ev.itemsize * 4 + 8), replace=False))
+        out["events_rows"] = rows.astype(np.float64)
+        ev = ev[rows]
+    out["events"] = ev
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def slomo_weights():
@@ -286,7 +313,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-cpu", action="store_true", help="development: skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the events, frame offsets and frame times of the last timed headline step to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "headline"):
+        ap.error("--dump-outputs writes the headline workload of --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -346,20 +379,23 @@ def main():
             dist.all_reduce(c, op=dist.ReduceOp.SUM)
         return t.item(), c.item()
 
-    def run_clips(src_host, src_dev, params, U_, batch, n_frames, rows_hint, steps, warmup, e2e, clip_seconds, seed):
+    def run_clips(src_host, src_dev, params, U_, batch, n_frames, rows_hint, steps, warmup, e2e, clip_seconds, seed,
+                  last_step=None):
         """`steps` timed passes of SloMo + pixel model over this rank's clip. Returns (ms max over ranks, events
-        summed over ranks, pipeline)."""
+        summed over ranks, pipeline). A `last_step` list receives host copies of the (events, offsets, times) the
+        last timed pass returned."""
         sl = SuperSloMo(model=None, auto_upsample=False, upsampling_factor=U_, batch_size=batch, device=devname,
                         state_dicts=wts)
         em = EventEmulator(device=devname, rng_mode="device", seed=seed, max_frames_per_step=n_frames, **params)
         em.event_rows_hint = rows_hint
         pipe = V2EPipeline(sl, em)
         k = 0
+        last = None
 
         period = clip_seconds * n_frames / (n_frames - 1)      # the next pass starts one frame interval after the last frame
 
         def one():
-            nonlocal k
+            nonlocal k, last
             t0 = k * period
             k += 1
             if e2e:
@@ -373,6 +409,7 @@ def main():
                 ev, offs, t, nf = pipe.run(src_dev, clip_seconds, t_offset=t0, return_device=True)
                 if world > 1:
                     gather_events(ev)
+            last = (ev, offs, t)
             return ev.shape[0]
         for _ in range(warmup):
             one()
@@ -384,6 +421,9 @@ def main():
             n += one()
         e1.record()
         barrier()
+        if last_step is not None:
+            ev, offs, t = last          # rows are views of buffers the next pass reuses: copy them now
+            last_step.extend([ev.cpu().numpy() if torch.is_tensor(ev) else np.array(ev), np.array(offs), np.array(t)])
         ms, cnt = all_max_sum(e0.elapsed_time(e1), n)
         return ms, cnt, pipe
 
@@ -477,9 +517,12 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
+    last_step = [] if args.dump_outputs and rank == 0 else None
     ms_dev, ev_dev, pipe = run_clips(src_host, src_dev, CLI_DEFAULTS, U, args.batch, n_interp, 48 * 1024 * 1024,
-                                     args.steps, args.warmup, False, clip_s, 1234 + rank)
+                                     args.steps, args.warmup, False, clip_s, 1234 + rank, last_step)
     clocks = sampler.stop() if rank == 0 else None
+    if last_step:
+        dump_outputs(args.dump_outputs, *last_step)
     _a, _b = ctypes.c_longlong(0), ctypes.c_longlong(0)
     pipe.emulator._lib.v2e_emu_fused_stats(pipe.emulator._h, ctypes.byref(_a), ctypes.byref(_b))
     _c, _d = ctypes.c_int(0), ctypes.c_int(0)
