@@ -58,6 +58,51 @@ class TapeRNG:
         return self.pos == len(self.tape)
 
 
+def smooth_background(H, W, T, seed=0, lo=90.0, hi=150.0):
+    """Smooth low-contrast texture translating 1 px per frame: 0-2 events per pixel and frame at
+    thresholds 0.05 (0-1 at 0.2)."""
+    from bench import source_clip
+    return source_clip(H, W, 2 * T + 1, seed=seed, px_per_frame=1, up=8, lo=lo, hi=hi)[:T]
+
+
+def patch_codes(targets, th=0.05, cutoff_hz=0.0, dt=2.0 ** -6, start=30):
+    """uint8 codes of one pixel, frame by frame, such that the CPU oracle (scalar threshold `th`, no noise, no
+    refractory period) makes exactly targets[k] events in frame k. Frame 0 initialises the state. A target of 0
+    keeps the code (the residual left after the last step is below one threshold); any other target is searched
+    upwards from the current code, then downwards."""
+    import copy
+    from emu_oracle import OracleEmulator
+    o = OracleEmulator(pos_thres=th, neg_thres=th, sigma_thres=0.0, cutoff_hz=cutoff_hz, leak_rate_hz=0.0,
+                       shuffle=False)
+    px = lambda c: np.full((1, 1), c, np.uint8)
+    o.generate_events(px(start), 0.0)
+    codes, code = [start], start
+    for k, n in enumerate(targets[1:], 1):
+        cands = [code] if n == 0 else list(range(code + 1, 256)) + list(range(code - 1, -1, -1))
+        for c in cands:
+            trial = copy.deepcopy(o)
+            trial.generate_events(px(c), k * dt)
+            if trial.last_max_n == n:
+                break
+        else:
+            raise ValueError("no code makes %d events in frame %d" % (n, k))
+        o.generate_events(px(c), k * dt)
+        codes.append(c)
+        code = c
+    return codes
+
+
+def scripted_clip(H, W, T, patches, th=0.05, cutoff_hz=0.0, dt=2.0 ** -6, seed=0, lo=90.0, hi=150.0):
+    """Smooth background plus small square patches whose level steps so that each patch pixel makes a chosen
+    number of events per frame. patches: [(y, x, size, targets, start_code)], targets[k] for frame k (length T)."""
+    fr = smooth_background(H, W, T, seed=seed, lo=lo, hi=hi).copy()
+    for y, x, s, targets, start in patches:
+        assert len(targets) == T
+        codes = patch_codes(targets, th=th, cutoff_hz=cutoff_hz, dt=dt, start=start)
+        fr[:, y:y + s, x:x + s] = np.asarray(codes, np.uint8)[:, None, None]
+    return fr
+
+
 def split_events(events, counts):
     off = np.concatenate([[0], np.cumsum(counts)])
     return [events[off[i]:off[i + 1]] for i in range(len(counts))]

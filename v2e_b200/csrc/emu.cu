@@ -2875,7 +2875,8 @@ extern "C" int v2e_emu_collect(V2eEmu *h, V2eFrameInfo *info, int T, int *frames
         CU(cudaStreamSynchronize(st));
     }
     int status = h->abort_host[0], done = status ? h->abort_host[1] : T;
-    if (!status && h->last_fused == 1 && h->n_seg == 1) h->fused_penalty = 0;       // a whole chunk accepted
+    // a whole chunk accepted (a rejected chunk can also end as one segment: frame by frame, which is no reset)
+    if (!status && h->last_fused == 1 && h->n_seg == 1 && h->sched[0].kind == 0) h->fused_penalty = 0;
     if (!status && h->last_fused == 1 && h->n_seg > 0) {
         for (int k = 0; k < h->n_seg; k++)
             (h->sched[k].kind == 0 ? h->n_frames_multi : h->n_frames_single) += h->sched[k].b - h->sched[k].a;
